@@ -63,7 +63,12 @@ def parse():
     ap.add_argument("--no-fusion", action="store_true")
     ap.add_argument("--mega", action="store_true", help="experimental: attention as a phase of the persistent decode kernel")
     ap.add_argument("--mega-mmv", action="store_true", help="experimental: attention and the matvecs inside the persistent decode kernel")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (logits f32, next token) as DIR/<name>.npy; "
+                    "the inputs are seeded, so two builds can be compared output for output (N = 1 only)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.gpus > 1:
+        ap.error("--dump-outputs is supported for --gpus 1 only")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -320,7 +325,7 @@ def run_b200(args):
     stream = torch.cuda.Stream()
     hbm_peak, peak_src = peaks()
 
-    res = device_resident_leg(args, model, ex, ops, G, stream, flags, args.n_past, args.steps, args.warmup, local, clocks=True)
+    res = device_resident_leg(args, model, ex, ops, G, stream, flags, args.n_past, args.steps, args.warmup, local, clocks=True, dump_dir=args.dump_outputs)
     tps, ms_per_step = res["tps"], res["ms_per_step"]
 
     # ---- roofline leg: the matvec launches of the step, in situ
@@ -403,8 +408,9 @@ def n_kv_of(pos):
     return max(256, (pos + 1 + 255) // 256 * 256)
 
 
-def device_resident_leg(args, model, ex, ops, G, stream, flags, n_past, steps, warmup, local, clocks):
-    """`value`: every input already in HBM — 3 tiny D2D copies + the token graph + on-device argmax feeding the next step"""
+def device_resident_leg(args, model, ex, ops, G, stream, flags, n_past, steps, warmup, local, clocks, dump_dir=None):
+    """`value`: every input already in HBM — 3 tiny D2D copies + the token graph + on-device argmax feeding the next step.
+    dump_dir: where to write the last timed step's logits and next token (see dump_outputs)"""
     import torch
     c = model.c
     V = c["n_vocab"]
@@ -440,6 +446,7 @@ def device_resident_leg(args, model, ex, ops, G, stream, flags, n_past, steps, w
         io["mask"][0].copy_(mask_dev[i], non_blocking=True)
         ex.compute(nodes, flags, stream=C.c_void_p(stream.cuda_stream))
         ops.check(ops.lib.b200_argmax_f32(ops.p(io["logits"]), ops.p(io["tokens"]), V, 1, C.c_void_p(stream.cuda_stream)))
+        return io
 
     with torch.cuda.stream(stream):
         for i in range(total + 1):
@@ -461,15 +468,26 @@ def device_resident_leg(args, model, ex, ops, G, stream, flags, n_past, steps, w
         torch.cuda.synchronize()
         e0.record(stream)
         for i in range(warmup, total):
-            device_step(i)
+            last_io = device_step(i)
         e1.record(stream)
         torch.cuda.synchronize()
         launches = ops.lib.b200_kernel_launches() - l0
         ms = e0.elapsed_time(e1)
         clk = sampler.stop() if sampler else None
+    if dump_dir and steps > 0:
+        dump_outputs(dump_dir, last_io)
     ms_per_step = ms / steps
     return {"tps": 1000.0 / ms_per_step, "ms_per_step": ms_per_step, "launches": launches, "kernels_per_step": ex.last_kernels + 1, "clocks": clk,
             "weight_bytes": model.streamed_weight_bytes(), "kv_bytes_per_pos": model.kv_bytes_per_pos(), "n_kv_mid": n_kv_of(n_past + warmup + steps // 2), "n_layer": len(model.layers)}
+
+
+def dump_outputs(out_dir, io):
+    """What a caller of the timed decode step receives: the logits of the step (f32 [1, n_vocab], 0.5 MB for Llama-3's
+    vocabulary) and the greedy next token the on-device argmax fed back (as f64, exact).  Written after the timing."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), io["logits"].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "next_token.npy"), io["tokens"].cpu().numpy().astype(np.float64))
 
 
 def mmvq_roofline_insitu(args, model, ex, ops, G, stream, flags, hbm_peak):
