@@ -193,6 +193,19 @@ B200_API int b200_mul_mat_vec_wide(int type, const void *W, const float *x, int6
 B200_API int b200_mul_mat_id(int type, const void *as, int64_t expert_stride_bytes, const float *b, int64_t b_tok_stride, int64_t b_slot_stride, int64_t n_b1,
                              const int32_t *ids, int64_t ids_tok_stride, float *dst, int64_t dst_tok_stride, int64_t dst_slot_stride,
                              int64_t m, int64_t k, int64_t n_expert, int64_t n_used, int64_t n_tok, void *stream);
+/* MUL_MAT_ID for prefill: the same contract and arguments as b200_mul_mat_id, plus a workspace.  For ubatches of at least 9 tokens
+ * with at least 4 (token, slot) pairs per expert (n_tok * n_used >= 4 * n_expert: where it measured faster) on Q4_K / Q5_K / Q6_K experts whose shape the tensor-core MUL_MAT takes (b200_mul_mat_q: k % 256 == 0, Q6_K k % 2048 == 0, not
+ * switched off by B200_MMQ_DISABLE_TC), with n_expert <= 256, n_tok * n_used <= 16384 and b200_mul_mat_id's alignment rules, it runs
+ * three kernels: a routing kernel groups the (token, slot) pairs by expert ON THE DEVICE (stable: increasing (t, s) inside an expert;
+ * ids outside [0, n_expert) dropped), the activations are quantised to q8_K gathered in that order, and the tensor-core GEMM reads
+ * each expert's weights once per 128 pairs.  Every other call is exactly b200_mul_mat_id.  No device->host synchronisation (the
+ * reference sorts on the host: ggml-cuda/mmq.cu:145-228), so a captured CUDA graph stays valid when the ids change between replays.
+ * b200_mul_mat_id_q_workspace returns 0 exactly when the call takes b200_mul_mat_id (workspace may then be NULL); otherwise the
+ * workspace (256-byte aligned) must hold that many bytes. */
+B200_API int64_t b200_mul_mat_id_q_workspace(int type, int64_t m, int64_t k, int64_t n_expert, int64_t n_used, int64_t n_tok);
+B200_API int b200_mul_mat_id_q(int type, const void *as, int64_t expert_stride_bytes, const float *b, int64_t b_tok_stride, int64_t b_slot_stride, int64_t n_b1,
+                               const int32_t *ids, int64_t ids_tok_stride, float *dst, int64_t dst_tok_stride, int64_t dst_slot_stride,
+                               int64_t m, int64_t k, int64_t n_expert, int64_t n_used, int64_t n_tok, void *workspace, void *stream);
 /* GET_ROWS on a quantised table: dst row i = de-quantised row ids[i] of src (replaces k_get_rows, ggml-cuda/getrows.cu:5-67; values
  * bit-identical to ggml's dequantize_row_*: products rounded separately).  The token-embedding lookup on the device. */
 B200_API int b200_get_rows_q(int type, const void *src, int64_t src_row_stride_bytes, int64_t nrows, const int32_t *ids, float *dst,

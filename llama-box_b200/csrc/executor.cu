@@ -941,11 +941,17 @@ struct Runner {
                 invalidate_act(n.dst);
                 return KL(b200_sum_rows((const float *)n.src[0].data, n.src[0].ne[0], (float *)n.dst.data, n.src[0].ne[0], nrows_of(n.src[0]), st));
             case B200_OP_MUL_MAT_ID: {
-                // expert routing on the device: the kernel reads ids itself (no stream synchronisation, unlike ggml-cuda.cu:2115-2125)
+                // expert routing on the device: the kernels read ids themselves (no stream synchronisation, unlike ggml-cuda.cu:2115-2125).
+                // Prefill ubatches take the grouped tensor-core path (3 launches, its workspace is the q8_K act buffer); decode / verify
+                // batches the one-launch matvec of b200_mul_mat_id
                 invalidate_act(n.dst);
                 const b200_tensor & w = n.src[0], & x = n.src[1], & ids = n.src[2];
-                return KL(b200_mul_mat_id(w.type, w.data, w.nb[2], (const float *)x.data, x.nb[2] / 4, x.nb[1] / 4, x.ne[1], (const int32_t *)ids.data, ids.nb[1] / 4,
-                                          (float *)n.dst.data, n.dst.nb[2] / 4, n.dst.nb[1] / 4, w.ne[1], w.ne[0], w.ne[2], ids.ne[0], ids.ne[1], st));
+                if (b200_mul_mat_id_q_workspace(w.type, w.ne[1], w.ne[0], w.ne[2], ids.ne[0], ids.ne[1]) > 0) {
+                    ex->act_id[0] = ex->act_id[1] = 0;       // the grouped path owns the act buffers
+                    if (dry) planned += 2;                   // routing + gathered quantisation ahead of the GEMM
+                }
+                return KL(b200_mul_mat_id_q(w.type, w.data, w.nb[2], (const float *)x.data, x.nb[2] / 4, x.nb[1] / 4, x.ne[1], (const int32_t *)ids.data, ids.nb[1] / 4,
+                                            (float *)n.dst.data, n.dst.nb[2] / 4, n.dst.nb[1] / 4, w.ne[1], w.ne[0], w.ne[2], ids.ne[0], ids.ne[1], act_buf(0), st));
             }
             case B200_OP_GET_ROWS:
                 invalidate_act(n.dst);
@@ -1012,6 +1018,9 @@ int plan_workspace(b200_executor * ex, const b200_node * nodes, int n) {
                 const size_t b = (size_t)b200_mul_mat_q_workspace(nd.src[0].type, nd.src[0].ne[1], k, cols);
                 if (kd >= 0 && b > act[kd]) act[kd] = b;
             }
+        } else if (nd.op == B200_OP_MUL_MAT_ID && nd.n_src >= 3) {   // grouped prefill path: routing + the gathered B image
+            const size_t b = (size_t)b200_mul_mat_id_q_workspace(nd.src[0].type, nd.src[0].ne[1], nd.src[0].ne[0], nd.src[0].ne[2], nd.src[2].ne[0], nd.src[2].ne[1]);
+            if (b > act[0]) act[0] = b;
         } else if (nd.op == B200_OP_RMS_NORM) {
             for (int kd = 0; kd < 2; kd++) { const size_t b = (size_t)(8 * act_col_bytes(kd, (nd.src[0].ne[0] + 255) / 256 * 256)); if (b > act[kd]) act[kd] = b; }
         } else if (nd.op == B200_OP_FLASH_ATTN_EXT) {

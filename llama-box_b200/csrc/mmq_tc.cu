@@ -35,86 +35,16 @@
 // imin operands + scale rings, ~200 KB.  Data movement: weights are read from HBM once per 128-token tile (L2 serves the
 // other token tiles of the same rows, which run on neighbouring CTAs), activations stream from L2.
 #include "common.cuh"
+#include "mmq_quant.cuh"          // TcGeom / tc_geom, quantize_mmq_kernel (the B image), MoeTile
 
 #include <cuda_fp16.h>
 #include <cstdio>
 #include <cstdlib>
 
 #define TC_TM 128
-#define TC_TN 128
 #define TC_THREADS 448
 #define TC_STAGE_A 32768
 #define TC_STAGE_B 32768
-#define TC_PANEL 2048             // one K-chunk (8 f16 = 16 bytes) of 128 rows
-
-// ---- workspace geometry (the B image) ------------------------------------------------------------------------------
-// per 128-token tile nt: Bq[nt][kq = k/64][chunk 0..7][n 0..127][8 f16]   (16 KB per 64-k quarter)
-//                        Bm[nt][sb][chunk 0..1][n][8 f16]                  (q8_K bsums, 4 KB per super-block)
-//                        D8[nt][sb][n] f32                                 (512 B per super-block)
-struct TcGeom { int64_t nt, kq, nsb, off_bq, off_bm, off_d8, total; };
-static TcGeom tc_geom(int64_t k, int64_t ncols) {
-    TcGeom g;
-    g.nt = (ncols + TC_TN - 1) / TC_TN; g.kq = k / 64; g.nsb = k / 256;
-    g.off_bq = 0;
-    g.off_bm = g.nt * g.kq * 16384;
-    g.off_d8 = g.off_bm + g.nt * g.nsb * 4096;
-    g.total  = g.off_d8 + g.nt * g.nsb * 512;
-    return g;
-}
-
-// ---- activation quantisation into the B image -------------------------------------------------------------------------
-// one warp per (token, super-block); exactly quantize_row_q8_K_ref: first index of the largest |x|, iscale = -127/max,
-// nearest-int (RNE), MIN(127, .), d = 1/iscale, bsums per 16
-__global__ void __launch_bounds__(256) quantize_mmq_kernel(const float * __restrict__ x, int64_t x_col_stride, int64_t ncols, int64_t k,
-                                                          uint8_t * __restrict__ ws, TcGeom g) {
-    pdl_wait();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t sb = blockIdx.x;
-    const int64_t n = (int64_t)blockIdx.y * 8 + warp;                // token (padded range: < nt * 128)
-    const int64_t nt = n >> 7; const int nl = (int)(n & 127);
-    float v[8] = { 0, 0, 0, 0, 0, 0, 0, 0 };
-    if (n < ncols) {
-        const float4 * p = (const float4 *)(x + n * x_col_stride + sb * 256 + lane * 8);
-        const float4 a = p[0], b = p[1];
-        v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
-    }
-    float am = 0.0f; int ai = 0;
-#pragma unroll
-    for (int j = 0; j < 8; j++) { const float a = fabsf(v[j]); if (a > am) { am = a; ai = lane * 8 + j; } }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const float am2 = __shfl_xor_sync(0xffffffffu, am, o);
-        const int   ai2 = __shfl_xor_sync(0xffffffffu, ai, o);
-        if (am2 > am || (am2 == am && ai2 < ai)) { am = am2; ai = ai2; }
-    }
-    float mine = 0.0f;
-#pragma unroll
-    for (int j = 0; j < 8; j++) if ((ai & 7) == j) mine = v[j];
-    const float maxv = __shfl_sync(0xffffffffu, mine, ai >> 3);
-    int q[8]; int s = 0; float d = 0.0f;
-    if (am != 0.0f) {
-        const float iscale = __fdiv_rn(-127.0f, maxv);
-#pragma unroll
-        for (int j = 0; j < 8; j++) { const int t = __float2int_rn(__fmul_rn(iscale, v[j])); q[j] = t > 127 ? 127 : t; s += q[j]; }
-        d = __fdiv_rn(1.0f, iscale);
-    } else {
-#pragma unroll
-        for (int j = 0; j < 8; j++) q[j] = 0;
-    }
-    // 8 consecutive elements = one K-chunk of the panel; element order inside a chunk is (0,2,1,3,4,6,5,7): the order in
-    // which the weight transform extracts nibbles from a 32-bit word (see unpack in the GEMM kernel)
-    auto h2 = [](int a, int b) { return (uint32_t)__half_as_ushort(__int2half_rn(a)) | ((uint32_t)__half_as_ushort(__int2half_rn(b)) << 16); };
-    uint4 pk; pk.x = h2(q[0], q[2]); pk.y = h2(q[1], q[3]); pk.z = h2(q[4], q[6]); pk.w = h2(q[5], q[7]);
-    const int64_t kq = sb * 4 + (lane >> 3); const int c = lane & 7;
-    *(uint4 *)(ws + g.off_bq + ((nt * g.kq + kq) * 8 + c) * TC_PANEL + nl * 16) = pk;
-    s += __shfl_xor_sync(0xffffffffu, s, 1);                          // bsum of 16 elements (|.| <= 2032: exact in f16)
-    if ((lane & 1) == 0) {
-        const int grp = lane >> 1;
-        *(__half *)(ws + g.off_bm + ((nt * g.nsb + sb) * 2 + (grp >> 3)) * TC_PANEL + nl * 16 + (grp & 7) * 2) = __int2half_rn(s);
-    }
-    if (lane == 0) *(float *)(ws + g.off_d8 + ((nt * g.nsb + sb) * 128 + nl) * 4) = d;
-    pdl_trigger();
-}
 
 // ---- tcgen05 / TMEM primitives (inline PTX; SASS: UTCHMMA, LDTM, UTCBAR, ...) -------------------------------------------
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -154,6 +84,10 @@ struct TcArgs {
     int32_t nsb, n_mtiles, n_tiles, type;
     uint32_t lbo, sbo;          // descriptor strides (bytes): K-chunk stride / 8-row-group stride
     unsigned long long * prof;  // bring-up: per-role cycle counters of CTA 0 (B200_MMQ_PROF), normally null
+    // grouped instances (MUL_MAT_ID) only: the routing of moe_route_kernel; column c of group tile g is pair
+    // gperm[gtiles[g].first + c] = (t, s), weights of expert gtiles[g].expert at W + expert * expert_stride
+    const MoeTile * gtiles; const int32_t * gperm; const int32_t * n_gtiles;
+    int64_t expert_stride, dst_tok_stride, dst_slot_stride;
 };
 // wait on an mbarrier, optionally accounting the cycles to a profile counter
 __device__ __forceinline__ void mbar_wait_p(uint64_t * bar, uint32_t parity, unsigned long long * acc) {
@@ -196,7 +130,9 @@ __device__ __forceinline__ void k4_unpack(uint32_t y, uint32_t z, uint32_t w, ui
     mn47 = ((w >> 4) & 0x0f0f0f0fu) | (((z >> 6) & 0x03030303u) << 4);
 }
 
-template <int T>
+// GROUPED: work items are (m-tile, group tile) with the group-tile count read from device memory (*args.n_gtiles); items of one
+// (expert, m-tile) are adjacent, so concurrently running CTAs share weight rows through L2
+template <int T, bool GROUPED>
 __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_constant__ TcArgs args) {
     using TT = TcType<T>;
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -225,7 +161,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
     pdl_wait();
 
     const int nsb = args.nsb;
-    const int64_t NT = args.g.nt;
+    const int64_t NT = GROUPED ? (int64_t)*args.n_gtiles : args.g.nt;   // N tiles: group tiles are written by the routing kernel before this grid
+    const int n_tiles = GROUPED ? args.n_mtiles * (int)NT : args.n_tiles;
     unsigned long long w0 = 0, w1 = 0, w2 = 0;                       // profile: cycles in this role's three kinds of waits
     const bool prof = args.prof != nullptr && blockIdx.x == 0;
     unsigned long long * pw0 = prof ? &w0 : nullptr, * pw1 = prof ? &w1 : nullptr, * pw2 = prof ? &w2 : nullptr;
@@ -234,7 +171,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
     if (warp == 12) {
         // ===================== TMA producer: activation panels, one per stage (+ the bsum panel and d_x with the first) =====================
         uint32_t it = 0, sbc = 0;
-        for (int tile = blockIdx.x; tile < args.n_tiles; tile += gridDim.x) {
+        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             const int64_t nt = tile % NT;
             for (int sb = 0; sb < nsb; sb++, sbc++) {
                 const int rs = sbc & 1;
@@ -261,9 +198,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
         // ===================== MMA issuer (one thread) =====================
         if (lane == 0) {
             uint32_t it = 0, sbc = 0;
-            for (int tile = blockIdx.x; tile < args.n_tiles; tile += gridDim.x) {
+            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                 const int64_t nt = tile % NT;
-                const int64_t nval = args.ncols - nt * TC_TN < TC_TN ? args.ncols - nt * TC_TN : TC_TN;
+                const int64_t nval = GROUPED ? (int64_t)args.gtiles[nt].count : (args.ncols - nt * TC_TN < TC_TN ? args.ncols - nt * TC_TN : TC_TN);
                 const uint32_t n_eff = (uint32_t)((nval + 15) & ~15);
                 // instruction descriptor (cute::UMMA::InstrDescriptor): D = f32, A = B = f16, both K-major, N >> 3 at bit 17, M >> 4 at bit 24
                 const uint32_t idesc = (1u << 4) | ((n_eff >> 3) << 17) | ((uint32_t)(TC_TM >> 4) << 24);
@@ -307,7 +244,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
         auto fetch = [&](int tile, int sb) {
             const int64_t m0 = (int64_t)(tile / NT) * TC_TM;
             int64_t r = m0 + t; if (r >= args.m) r = args.m - 1;             // rows past the end: any valid row (their results are never stored)
-            const uint8_t * row = args.W + r * args.rb;
+            const uint8_t * W = GROUPED ? args.W + (int64_t)args.gtiles[tile % NT].expert * args.expert_stride : args.W;
+            const uint8_t * row = W + r * args.rb;
             if (T == B200_TYPE_Q6_K) {
                 const uint4 * ql = (const uint4 *)(row + (int64_t)sb * 128), * qh = (const uint4 *)(row + nb * 128 + (int64_t)sb * 64);
 #pragma unroll
@@ -322,8 +260,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
                 for (int i = 0; i < NW; i++) nxt[i] = __ldg(p + i);
             }
         };
-        if (blockIdx.x < args.n_tiles) fetch(blockIdx.x, 0);
-        for (int tile = blockIdx.x; tile < args.n_tiles; tile += gridDim.x) {
+        if (blockIdx.x < n_tiles) fetch(blockIdx.x, 0);
+        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             for (int sb = 0; sb < nsb; sb++, sbc++) {
                 const int rs = sbc & 1;                                  // accumulator / imin-operand slot
                 uint4 cur[NW]; const uint16_t cur_d = nxt_d;
@@ -332,7 +270,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
                 {   // prefetch the next super-block (of this tile, or the first one of this CTA's next tile)
                     int ntile = tile, nsbi = sb + 1;
                     if (nsbi == nsb) { nsbi = 0; ntile = tile + gridDim.x; }
-                    if (ntile < args.n_tiles) fetch(ntile, nsbi);
+                    if (ntile < n_tiles) fetch(ntile, nsbi);
                 }
                 float2 * rscale = (float2 *)(smem + TcSmem::RS + (sbc & 3) * 1024);
                 if (T == B200_TYPE_Q4_K || T == B200_TYPE_Q5_K) {
@@ -440,9 +378,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
         const int quad = warp & 3, ch = warp >> 2;
         const int r = quad * 32 + lane;                                   // tile row = TMEM lane
         uint32_t sbc = 0;
-        for (int tile = blockIdx.x; tile < args.n_tiles; tile += gridDim.x) {
+        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             const int64_t mt = tile / NT, nt = tile % NT;
-            const int64_t nval = args.ncols - nt * TC_TN < TC_TN ? args.ncols - nt * TC_TN : TC_TN;
+            MoeTile gt = {};
+            if (GROUPED) gt = args.gtiles[nt];
+            const int64_t nval = GROUPED ? (int64_t)gt.count : (args.ncols - nt * TC_TN < TC_TN ? args.ncols - nt * TC_TN : TC_TN);
             const int n_eff = (int)((nval + 15) & ~15);
             float acc[64];
 #pragma unroll
@@ -475,7 +415,18 @@ __global__ void __launch_bounds__(TC_THREADS, 1) mmq_tc_kernel(const __grid_cons
                 if (lane == 0) mbar_arrive(&acc_empty[rs]);
             }
             const int64_t row = mt * TC_TM + r;
-            if (row < args.m) {
+            if (GROUPED) {
+                if (row < args.m) {
+#pragma unroll
+                    for (int c = 0; c < 64; c++) {
+                        const int n = ch * 64 + c;
+                        if (n < gt.count) {                                // pair (t, s) of column n -> dst row block (t, s)
+                            const int32_t pr = args.gperm[gt.first + n];
+                            args.dst[(int64_t)(pr >> 16) * args.dst_tok_stride + (int64_t)(pr & 0xffff) * args.dst_slot_stride + row] = acc[c];
+                        }
+                    }
+                }
+            } else if (row < args.m) {
 #pragma unroll
                 for (int c = 0; c < 64; c++) {
                     const int64_t n = nt * TC_TN + ch * 64 + c;
@@ -506,12 +457,12 @@ bool b200_mmq_tc_supported(int type, int64_t m, int64_t k, int64_t ncols) {
 }
 int64_t b200_mmq_tc_workspace(int64_t k, int64_t ncols) { return tc_geom(k, ncols).total; }
 
-template <int T> static int tc_launch(const TcArgs & a, cudaStream_t st) {
+template <int T, bool GROUPED> static int tc_launch(const TcArgs & a, cudaStream_t st) {
     static bool attr[64] = { false };
     int dev = 0; cudaGetDevice(&dev);
-    if (!attr[dev & 63]) { B200_CUDA(cudaFuncSetAttribute(mmq_tc_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::TOTAL)); attr[dev & 63] = true; }
+    if (!attr[dev & 63]) { B200_CUDA(cudaFuncSetAttribute(mmq_tc_kernel<T, GROUPED>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::TOTAL)); attr[dev & 63] = true; }
     int grid = a.n_tiles < b200_sm_count() ? a.n_tiles : b200_sm_count();
-    B200_CUDA(b200_launch_pdl(mmq_tc_kernel<T>, dim3((unsigned)grid), dim3(TC_THREADS), (size_t)TcSmem::TOTAL, st, a));
+    B200_CUDA(b200_launch_pdl(mmq_tc_kernel<T, GROUPED>, dim3((unsigned)grid), dim3(TC_THREADS), (size_t)TcSmem::TOTAL, st, a));
     b200_count_launch();
     return B200_OK;
 }
@@ -530,13 +481,13 @@ int b200_mmq_tc(int type, const void * W, const float * X, int64_t x_col_stride,
     a.prof = want_prof ? prof_buf : nullptr;
     a.nsb = (int32_t)(k / 256); a.n_mtiles = (int32_t)((m + TC_TM - 1) / TC_TM); a.n_tiles = (int32_t)(a.n_mtiles * a.g.nt); a.type = type;
     dim3 qgrid((unsigned)a.nsb, (unsigned)(a.g.nt * 16));
-    B200_CUDA(b200_launch_pdl(quantize_mmq_kernel, qgrid, dim3(256), 0, st, X, x_col_stride, ncols, k, (uint8_t *)workspace, a.g));
+    B200_CUDA(b200_launch_pdl(quantize_mmq_kernel<false>, qgrid, dim3(256), 0, st, X, x_col_stride, ncols, k, (uint8_t *)workspace, a.g, TcGather{}));
     b200_count_launch();
     int rc = B200_ERR_UNSUPPORTED;
     switch (type) {
-        case B200_TYPE_Q4_K: rc = tc_launch<B200_TYPE_Q4_K>(a, st); break;
-        case B200_TYPE_Q5_K: rc = tc_launch<B200_TYPE_Q5_K>(a, st); break;
-        case B200_TYPE_Q6_K: rc = tc_launch<B200_TYPE_Q6_K>(a, st); break;
+        case B200_TYPE_Q4_K: rc = tc_launch<B200_TYPE_Q4_K, false>(a, st); break;
+        case B200_TYPE_Q5_K: rc = tc_launch<B200_TYPE_Q5_K, false>(a, st); break;
+        case B200_TYPE_Q6_K: rc = tc_launch<B200_TYPE_Q6_K, false>(a, st); break;
     }
     if (want_prof && rc == B200_OK) {
         unsigned long long h[16 * 4];
@@ -548,4 +499,63 @@ int b200_mmq_tc(int type, const void * W, const float * X, int64_t x_col_stride,
         fprintf(stderr, "  (epi: wait0 = acc_full | xform: wait1 = ab_empty | mma: wait0 = acc_empty, wait1 = b_full, wait2 = a_full | b-tma: wait0 = ab_empty)\n");
     }
     return rc;
+}
+
+// ---- grouped MUL_MAT_ID (b200_mul_mat_id_q): routing, gathered quantisation, grouped GEMM -----------------------------
+// workspace: [B image of moe_max_tiles group tiles][tile table][n_gtiles][perm], sections 256-byte aligned
+struct TcIdGeom { int64_t g_max, off_tiles, off_cnt, off_perm, total; TcGeom g; };
+static TcIdGeom tc_id_geom(int64_t k, int64_t n_expert, int64_t n_pairs) {
+    auto up = [](int64_t x) { return (x + 255) & ~(int64_t)255; };
+    TcIdGeom r;
+    r.g_max = moe_max_tiles(n_expert, n_pairs);
+    r.g = tc_geom(k, r.g_max * TC_TN);
+    r.off_tiles = up(r.g.total);
+    r.off_cnt = r.off_tiles + up(r.g_max * (int64_t)sizeof(MoeTile));
+    r.off_perm = r.off_cnt + 256;
+    r.total = r.off_perm + up(n_pairs * 4);
+    return r;
+}
+bool b200_mmq_tc_id_routable(int64_t n_expert, int64_t n_used, int64_t n_tok) {
+    return n_expert > 0 && n_expert <= MR_MAX_EXPERT && n_used > 0 && n_tok > 0 && n_used * n_tok <= MR_MAX_PAIRS;
+}
+int64_t b200_mmq_tc_id_workspace(int64_t k, int64_t n_expert, int64_t n_used, int64_t n_tok) { return tc_id_geom(k, n_expert, n_used * n_tok).total; }
+
+// arguments as b200_mul_mat_id (validated by the caller, b200_mul_mat_id_q); workspace: b200_mmq_tc_id_workspace bytes, 256-byte aligned
+int b200_mmq_tc_id(int type, const void * as, int64_t expert_stride_bytes, const float * b, int64_t b_tok_stride, int64_t b_slot_stride, int64_t n_b1,
+                   const int32_t * ids, int64_t ids_tok_stride, float * dst, int64_t dst_tok_stride, int64_t dst_slot_stride,
+                   int64_t m, int64_t k, int64_t n_expert, int64_t n_used, int64_t n_tok, void * workspace, void * stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!b200_mmq_tc_id_routable(n_expert, n_used, n_tok)) {
+        b200_set_error("mul_mat_id: grouped routing takes at most %d experts and %d (token, slot) pairs", MR_MAX_EXPERT, MR_MAX_PAIRS); return B200_ERR_UNSUPPORTED;
+    }
+    if (((uintptr_t)as | (uintptr_t)b | (uintptr_t)workspace) & 15 || (b_tok_stride & 3) || (b_slot_stride & 3) || (expert_stride_bytes & 15)) {
+        b200_set_error("mul_mat_id: pointers must be 16-byte aligned"); return B200_ERR_INVALID;
+    }
+    const TcIdGeom G = tc_id_geom(k, n_expert, n_used * n_tok);
+    uint8_t * ws = (uint8_t *)workspace;
+    MoeTile * tiles = (MoeTile *)(ws + G.off_tiles); int32_t * cnt = (int32_t *)(ws + G.off_cnt); int32_t * perm = (int32_t *)(ws + G.off_perm);
+    B200_CUDA(b200_launch_pdl(moe_route_kernel, dim3(1), dim3(MR_THREADS), 0, st, ids, ids_tok_stride, (int)n_expert, (int)n_used, (int)n_tok, perm, tiles, cnt));
+    b200_count_launch();
+    TcGather ga = {};
+    ga.perm = perm; ga.tiles = tiles; ga.n_gtiles = cnt; ga.slot_stride = b_slot_stride; ga.n_b1 = (int32_t)n_b1;
+    const dim3 qgrid((unsigned)(k / 256), (unsigned)(G.g_max * 16));
+    B200_CUDA(b200_launch_pdl(quantize_mmq_kernel<true>, qgrid, dim3(256), 0, st, b, b_tok_stride, (int64_t)0, k, ws, G.g, ga));
+    b200_count_launch();
+    TcArgs a = {};
+    a.W = (const uint8_t *)as; a.ws = ws; a.dst = dst; a.m = m; a.k = k; a.ncols = 0; a.ldd = 0;
+    a.rb = (k / 256) * type_block_bytes(type);
+    a.g = G.g;
+    a.lbo = (uint32_t)TC_PANEL; a.sbo = 128u;
+    a.nsb = (int32_t)(k / 256); a.n_mtiles = (int32_t)((m + TC_TM - 1) / TC_TM);
+    a.n_tiles = (int32_t)(a.n_mtiles * G.g_max);                              // upper bound: sizes the persistent grid; the kernel reads the real count
+    a.type = type;
+    a.gtiles = tiles; a.gperm = perm; a.n_gtiles = cnt;
+    a.expert_stride = expert_stride_bytes; a.dst_tok_stride = dst_tok_stride; a.dst_slot_stride = dst_slot_stride;
+    switch (type) {
+        case B200_TYPE_Q4_K: return tc_launch<B200_TYPE_Q4_K, true>(a, st);
+        case B200_TYPE_Q5_K: return tc_launch<B200_TYPE_Q5_K, true>(a, st);
+        case B200_TYPE_Q6_K: return tc_launch<B200_TYPE_Q6_K, true>(a, st);
+    }
+    b200_set_error("mul_mat_id: grouped path has no kernel for type %d", type);
+    return B200_ERR_UNSUPPORTED;
 }

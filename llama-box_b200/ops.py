@@ -88,6 +88,8 @@ SIGNATURES = {
     "b200_wide_row_bytes": (i64, [i32, i64]),
     "b200_mul_mat_vec_wide": (i32, [i32, vp, vp, i64, vp, i64, vp, vp, i64, i64, i64, vp]),
     "b200_mul_mat_id": (i32, [i32, vp, i64, vp, i64, i64, i64, vp, i64, vp, i64, i64, i64, i64, i64, i64, i64, vp]),
+    "b200_mul_mat_id_q_workspace": (i64, [i32, i64, i64, i64, i64, i64]),
+    "b200_mul_mat_id_q": (i32, [i32, vp, i64, vp, i64, i64, i64, vp, i64, vp, i64, i64, i64, i64, i64, i64, i64, vp, vp]),
     "b200_get_rows_q": (i32, [i32, vp, i64, i64, vp, vp, i64, i64, i64, vp]),
     "b200_binary_strided": (i32, [i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "b200_soft_max_rows": (i32, [vp, i64, vp, i64, i64, i64, f32, vp]),
